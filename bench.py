@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- images/sec of the VisualCloze denoising hot path on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload B|A|Bp|D|E]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload B|A|Bp|D|E] [--dump-outputs DIR]
 
 One "step" = one image of the workload: the flow-matching Euler loop over the FLUX-DiT (30 time points = 29 model
 evaluations for the 384 grid 2x3 layout, SURVEY.md section 8) plus the VAE decode of the query row, on synthetic
@@ -15,6 +15,10 @@ inputs of the reference's shapes with random-init weights of the reference's geo
   cpu_baseline   the CPU oracle port (the reference's algorithm, un-merged LoRA, bf16 autocast semantics) timed on
           the host cores on a bounded sample (1 double + 1 single block at full width and full token count),
           extrapolated to images/sec -- a reported baseline, not the target.
+
+`--dump-outputs DIR` writes what the last timed step returned -- the decoded query-row image tile, uint8 values, gathered over
+the replicas -- to DIR/query_row_image.npy as float32.  Inputs and weights come from fixed seeds, so two builds run with the
+same arguments can be compared output for output.
 
 `--impl reference` times the reference arm: the UNMODIFIED reference modules of oracle/_ref (DoubleStreamBlock /
 SingleStreamBlock of models/modules/layers.py with LoRA r=256, bf16 autocast, attention through SDPA because flash-attn is
@@ -254,6 +258,7 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="B", choices=list(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output to DIR/<name>.npy (float32)")
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp8", "fp8_all"],
                     help="bf16 = the reference's numerics (the headline); fp8 = opt-in e4m3 projections for the LayerNorm-fed Linears "
                          "(a separate line with its own tolerance contract, never the headline)")
@@ -261,6 +266,8 @@ def main():
                     help="N>1: 'replicas' = one image per GPU (throughput, weak scaling; the default and the contract's line); "
                          "'sp' = ONE image sharded by token rows over the N GPUs (latency, strong scaling; SURVEY.md 8f-2)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -352,6 +359,8 @@ def main():
         kw = {k: v.to(dev, non_blocking=True) for k, v in kw_h.items()}
         return finish(fn(x, model.forward, kw)[-1]).cpu()
 
+    last = [None]                     # what the most recent timed step returned
+
     def timed(step, k):
         if world > 1:
             dist.barrier()
@@ -359,7 +368,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            step()
+            last[0] = step()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -375,6 +384,10 @@ def main():
     ms = timed(step_resident, args.steps)
     launches = lib.vcb_launch_count()
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "query_row_image.npy"), last[0].float().cpu().numpy())
     step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
     h2d = x_h.numel() * x_h.element_size() + sum(v.numel() * v.element_size() for v in kw_h.values())

@@ -1,7 +1,8 @@
 """Pipeline parity (SURVEY.md 8 rows a-15, a-16): ``VisualClozeModel.process_images`` / ``.upsampling`` against a composition of
 oracle pieces (oracle/pipeline_oracle.py: reference-equivalent mask packing and cond concat, the UNMODIFIED reference
-``prepare_modified`` from oracle/_ref, sampler + model oracle, ``vae_oracle.decode``, query-row crop, SDEdit blend) on the
-same injected stub encoders.
+``prepare_modified``, sampler + model oracle, ``vae_oracle.decode``, query-row crop, SDEdit blend) on the same injected stub
+encoders.  The composition needs the reference's own ``prepare_modified``, so its sampler inputs and final images were run once
+on a B200 and stored in tests/golden/pipeline_small.pt (``python oracle/gen_golden_gpu.py``).
 
   packed ``img_cond``, ``img_ids``, noise tokens, ``txt`` / ``y`` / masks / guidance handed to the sampler   bit-exact
   final PIL images                                                                                           PSNR >= 35 dB
@@ -30,9 +31,16 @@ def _psnr(a, b):
 def rig():
     if not torch.cuda.is_available():
         pytest.skip("needs a GPU")
-    from oracle import flux_oracle as fo, ref_runner as rr, vae_oracle as vo
-    if not rr.available():
-        pytest.skip("oracle/_ref (the unmodified reference prepare_modified) is absent")
+    return _rig()
+
+
+@pytest.fixture(scope="module")
+def golden():
+    return torch.load(os.path.join(GOLDEN, "pipeline_small.pt"), weights_only=False)
+
+
+def _rig():
+    from oracle import flux_oracle as fo, vae_oracle as vo
     import visualcloze_b200.model as M
     from visualcloze_b200 import pipeline as P, vae as V
     g = torch.load(os.path.join(GOLDEN, "flux_small_b1.pt"), weights_only=False)
@@ -86,15 +94,45 @@ def _grid():
     return imgs
 
 
+TAPS = ("x", "cond", "img_ids", "txt", "txt_ids", "txt_mask", "y", "img_mask", "guidance")
+
+
 def _same_inputs(ours: dict, orc: dict):
-    for k in ("x", "cond", "img_ids", "txt", "txt_ids", "txt_mask", "y", "img_mask", "guidance"):
+    for k in TAPS:
         a, b = ours[k], orc[k]
         assert a.shape == b.shape and a.dtype == b.dtype, (k, a.shape, b.shape, a.dtype, b.dtype)
         assert torch.equal(a.cpu(), b.cpu()), f"{k}: packed sampler input differs from the reference composition"
 
 
-def test_process_images_matches_oracle_composition(rig):
+def _oracle_kwargs(rig):
+    return {k: rig[k] for k in ("t5", "clip", "encode", "flux_p", "flux_cfg", "vae_p", "vae_cfg")}
+
+
+def oracle_process_images(rig):
+    """The reference composition for test_process_images_matches_oracle_composition: (sampler inputs, [cropped result])."""
     from oracle import pipeline_oracle as po
+    pipe = rig["pipe"]
+    pipe.set_grid_size(2, 3)
+    cells, mask_position, _ = pipe._prepare_grid([[im.convert("RGB") if im is not None else None for im in row] for row in _grid()])
+    taps = {}
+    ref, query, _ = po.process_images(cells, mask_position, 2, 3, ["layout prompt", "task prompt", "content prompt"], 5, 30, 4,
+                                      device=torch.device("cuda"), taps=taps, **_oracle_kwargs(rig))
+    return {k: taps[k].cpu() for k in TAPS}, [np.asarray(im) for im in ref]
+
+
+def oracle_upsampling(rig):
+    """The reference composition for test_upsampling_matches_oracle_composition: (sampler inputs, result)."""
+    from PIL import Image
+    from oracle import pipeline_oracle as po
+    rng = np.random.RandomState(3)
+    img = Image.fromarray(rng.randint(0, 255, (64, 64, 3), dtype=np.uint8))
+    taps = {}
+    g2 = torch.Generator(device="cuda").manual_seed(11)
+    ref = po.upsampling(img, (80, 96), 30, 4, 0.4, g2, "a cat", device=torch.device("cuda"), taps=taps, **_oracle_kwargs(rig))
+    return {k: taps[k].cpu() for k in TAPS}, np.asarray(ref)
+
+
+def test_process_images_matches_oracle_composition(rig, golden):
     pipe = rig["pipe"]
     pipe.set_grid_size(2, 3)
     seen = []
@@ -103,24 +141,19 @@ def test_process_images_matches_oracle_composition(rig):
         out = pipe.process_images(_grid(), ["layout prompt", "task prompt", "content prompt"], seed=5, cfg=30, steps=4, is_upsampling=False)
     finally:
         pipe._make_sample_fn = orig
-    cells, mask_position, _ = pipe._prepare_grid([[im.convert("RGB") if im is not None else None for im in row] for row in _grid()])
-    taps = {}
-    kw = {k: rig[k] for k in ("t5", "clip", "encode", "flux_p", "flux_cfg", "vae_p", "vae_cfg")}
-    ref, query, _ = po.process_images(cells, mask_position, 2, 3, ["layout prompt", "task prompt", "content prompt"], 5, 30, 4,
-                                      device=torch.device("cuda"), taps=taps, **kw)
+    taps, ref = golden["process_images"]
     assert len(seen) == 1
     _same_inputs(seen[0], taps)
-    assert len(out) == len(ref) == 1 and out[0].size == ref[0].size == (64, 64)
+    assert len(out) == len(ref) == 1 and out[0].size == (64, 64) and ref[0].shape == (64, 64, 3)
     p = _psnr(out[0], ref[0])
     print(f"[pipeline] process_images PSNR vs oracle composition: {p:.1f} dB")
     assert p >= 35.0, f"PSNR {p:.1f} dB"
 
 
-def test_upsampling_matches_oracle_composition(rig):
+def test_upsampling_matches_oracle_composition(rig, golden):
     """SDEdit second stage: blend ``noise * (1 - s) + latent * s`` (visualcloze.py:221), all-ones mask over a blank condition,
     1x1 grid, do_shift=False schedule from ``strength``."""
     from PIL import Image
-    from oracle import pipeline_oracle as po
     pipe = rig["pipe"]
     rng = np.random.RandomState(3)
     img = Image.fromarray(rng.randint(0, 255, (64, 64, 3), dtype=np.uint8))
@@ -132,13 +165,10 @@ def test_upsampling_matches_oracle_composition(rig):
                               content_prompt="The last image of the last row depicts: a cat")
     finally:
         pipe._make_sample_fn = orig
-    taps = {}
-    kw = {k: rig[k] for k in ("t5", "clip", "encode", "flux_p", "flux_cfg", "vae_p", "vae_cfg")}
-    g2 = torch.Generator(device="cuda").manual_seed(11)
-    ref = po.upsampling(img, (80, 96), 30, 4, 0.4, g2, "a cat", device=torch.device("cuda"), taps=taps, **kw)
+    taps, ref = golden["upsampling"]
     assert len(seen) == 1
     _same_inputs(seen[0], taps)
-    assert out.size == ref.size == (80, 96)
+    assert out.size == (80, 96) and ref.shape == (96, 80, 3)
     p = _psnr(out, ref)
     print(f"[pipeline] upsampling PSNR vs oracle composition: {p:.1f} dB")
     assert p >= 35.0, f"PSNR {p:.1f} dB"
